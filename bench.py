@@ -2,6 +2,7 @@
 
   python bench.py --gpus N --steps K --warmup W            (N > 1: launched by torchrun, one rank per GPU)
   python bench.py --impl reference ...                      (the unmodified reference; see DESIGN.md)
+  python bench.py ... --dump-outputs DIR                    (also write the last timed update's outputs; see dump_outputs)
 
 Batch: the default is ``--mini-batches 8`` = 4 x 8 x 8 = 256 prompts (x 4 samples = 1024 sequences) per rank per update
 -- the reference's arithmetic with ``num_mini_batches`` halved from 16 -- so that the driver's ``--steps 20 --warmup 5`` (25 full
@@ -55,7 +56,52 @@ def parse():
     ap.add_argument("--reward", default="deberta-large", choices=["deberta-large", "deberta-tiny"])
     ap.add_argument("--grad-checkpointing", type=int, default=0,
                     help="1 = recompute activations like the reference (A100-40G memory saver); 0 = keep them (B200: 180 GB)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed update computed to DIR/<name>.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+# Per-token arrays of the dump keep at most this many elements each (a seeded sample of rows beyond it), so that the four of
+# them plus the weight sample stay under 64 MB at any batch or response length.
+DUMP_TOKENS_PER_ARRAY = 2_500_000
+DUMP_SAMPLES_PER_WEIGHT = 2048
+
+
+def dump_outputs(out_dir, metrics, rollout, policy):
+    """Write what one update computed as ``out_dir/<name>.npy`` (float32 / float64) so that two builds can be compared on the
+    same seeded inputs: its metrics without timings (``metrics.*``, 0-d float64); the rollout it trained on -- ``responses``
+    (token ids), ``logprobs`` / ``ref_logprobs`` (policy / reference log-probs of those tokens), ``advantages``, ``scores``
+    (reward-model score) and ``normalized_scores`` (group-normalised), one row per sequence, the same seeded rows in each
+    when the batch is larger than the limit; and ``trainable_weights_sample``, a fixed seeded sample of every trainable
+    tensor of the updated policy, in name order."""
+    import numpy as np
+    import torch
+
+    out = {"metrics." + k.replace("/", "."): np.float64(v) for k, v in sorted(metrics.items())
+           if not k.startswith(("time/", "throughput/", "mem/"))}
+    n, t = rollout["responses"].shape
+    keep = max(1, DUMP_TOKENS_PER_ARRAY // t)
+    rows = torch.arange(n) if n <= keep else torch.randperm(n, generator=torch.Generator().manual_seed(0))[:keep].sort().values
+    for name, key in (("responses", "responses"), ("logprobs", "logprobs"), ("ref_logprobs", "ref_logprobs"),
+                      ("advantages", "advantages"), ("scores", "log_scores"), ("normalized_scores", "scores")):
+        x = rollout[key]
+        out[name] = x[rows.to(x.device)].float().cpu().numpy()
+    g = torch.Generator().manual_seed(0)
+    parts = []
+    for _, p in sorted(policy.named_parameters(), key=lambda kv: kv[0]):
+        if p.requires_grad:
+            flat = p.detach().reshape(-1)
+            idx = torch.randint(0, flat.numel(), (min(flat.numel(), DUMP_SAMPLES_PER_WEIGHT),), generator=g)
+            parts.append(flat[idx.to(flat.device)].float().cpu())
+    out["trainable_weights_sample"] = torch.cat(parts).numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    for name, arr in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
+    total = sum(a.nbytes for a in out.values())
+    print(f"[bench] wrote {len(out)} arrays ({total / 1e6:.1f} MB) to {out_dir}", file=sys.stderr, flush=True)
 
 
 def reference_arm(args):
@@ -131,6 +177,16 @@ def main():
     dataset = synthetic_token_dataset(prompts_per_rank * comm.world_size * 2, shape.vocab_size - 2, 24, 160, seed=1)
     trainer = GRPOTrainer(cfg, tok, policy, ref_policy, dataset, reward_func=reward, comm=comm)
     it = iter(trainer.dataloader)
+    rollout = {}
+    if args.dump_outputs:
+        # keep a reference to each update's rollout batch; it is copied to the host only after the timed region
+        algo_advantages = trainer.advantages
+
+        def advantages(R):
+            adv, ret = algo_advantages(R)
+            rollout.update(R, advantages=adv)
+            return adv, ret
+        trainer.advantages = advantages
 
     def one_update(u):
         batch = next(it)                                    # host tensors (collated, pinned by the trainer)
@@ -222,6 +278,8 @@ def main():
                                   "capture_failures": getattr(getattr(trainer, "_graphed", None), "capture_failures", 0)},
         }
         print(json.dumps(line), flush=True)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, m, rollout, trainer.policy)
     trainer.heartbeat.close()
     comm.barrier()
     comm.close()

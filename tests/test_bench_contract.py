@@ -4,6 +4,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -40,3 +41,27 @@ def test_bench_line_on_a_tiny_model():
     assert line["e2e"]["value"] <= line["value"] * 1.001          # wall clock around the same steps cannot beat the device time
     assert line["gpu_launches"] > 100
     assert set(line["clocks"]) >= {"sm_mhz", "sm_max_mhz", "reasons"}
+
+
+@pytest.mark.gpu
+def test_bench_dumps_the_last_timed_update(tmp_path):
+    """``--dump-outputs``: after exactly ``--steps`` timed updates, the last one's rollout, metrics and a weight sample land in
+    float32 / float64 ``.npy`` files of at most 64 MB in all."""
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--model", "tiny", "--reward", "deberta-tiny", "--response-length", "48",
+                        "--mini-batches", "1", "--steps", "2", "--warmup", "1", "--dump-outputs", str(tmp_path)],
+                       capture_output=True, text=True, timeout=900)
+    assert r.returncode == 0, r.stderr[-3000:]
+    line = _last_json(r.stdout)
+    assert len([ln for ln in r.stderr.splitlines() if ln.startswith("[bench] step ")]) == 2 and line["steps"] == 2
+    arrays = {f[:-len(".npy")]: np.load(tmp_path / f) for f in os.listdir(tmp_path)}
+    assert all(a.dtype in (np.float32, np.float64) for a in arrays.values())
+    assert sum(a.nbytes for a in arrays.values()) <= 64e6
+    rows = arrays["responses"].shape[0]
+    assert rows > 0 and arrays["responses"].shape == (rows, 48)
+    for k in ("logprobs", "ref_logprobs", "advantages"):
+        assert arrays[k].shape == (rows, 48) and np.isfinite(arrays[k]).all(), k
+    assert arrays["scores"].shape == arrays["normalized_scores"].shape == (rows,)
+    assert (arrays["responses"] == np.round(arrays["responses"])).all() and (arrays["responses"] >= 0).all()
+    assert arrays["trainable_weights_sample"].size > 0 and np.isfinite(arrays["trainable_weights_sample"]).all()
+    assert {"metrics.loss.policy_avg_new", "metrics.objective.kl_old"} <= set(arrays)
+    assert not any(k.startswith(("metrics.time.", "metrics.throughput.")) for k in arrays)

@@ -36,7 +36,8 @@ def build(cls, tmp_path, extra=None, reward=None, lora=True, **kw):
     if cls is PPOTrainer:
         vm = Qwen2ForSequenceClassification.from_causal_lm(ref)
         kwargs["value_model"] = get_peft_model(vm, LoraConfig(r=4, lora_alpha=8, modules_to_save=["score"]))
-    return cls(a, tok, policy, ref, ds, reward_func=reward or LengthReward(6), **kwargs)
+    # the PyTorch plumbing path on every machine, a GPU present or not (the CUDA runs are in test_trainers_gpu.py)
+    return cls(a, tok, policy, ref, ds, reward_func=reward or LengthReward(6), device=torch.device("cpu"), **kwargs)
 
 
 @pytest.mark.parametrize("cls,extra,kw", [
